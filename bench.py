@@ -19,6 +19,10 @@ computes; BASELINE configs[2] asks for levels 0-3, a subset) of ONE n^3 grid (n 
           region, every step.
 Inputs (1 GiB per channel at 1024^3) are far larger than the 126 MB L2, so no explicit L2 flush is needed.
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR (N = 1) writes what the last timed step computed, as a caller of vxb_polygonize receives it, to
+DIR/<name>.npy (see dump_outputs); the seeded terrain makes the inputs identical from run to run, so two builds can be
+compared output for output.
 """
 import os
 import sys
@@ -60,7 +64,51 @@ def parse_args():
     ap.add_argument("--group-planes", type=int, default=0, help="N > 1: planes per scan group / cube piece (0 = default)")
     ap.add_argument("--shard-mode", default="replicated", choices=["replicated", "cube"],
                     help="N > 1: volumes replicated in every rank's HBM (work sharded; default) or sharded as a peer-mapped cube")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1: write the last timed step's result to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs writes the result of one GPU (N = 1)")
+    return args
+
+
+# rows kept per array by --dump-outputs (136, 72, 8, 72 and 8 bytes a row): at most 56 MiB in all
+DUMP_ROWS = {"blocks": 1 << 17, "vertices": 1 << 18, "indices": 1 << 20, "transition_vertices": 1 << 17, "transition_indices": 1 << 19}
+
+
+def dump_outputs(res, directory):
+    """The result of one vxb_polygonize as float arrays, in the reference's order (levels, then blocks by coordinate, each
+    block's vertices and indices in turn; arena offsets, which vary from run to run, are left out):
+      blocks [B, 17] float64      level, coord_id, id, vertex_count, index_count, trans_vertex_count[6], trans_index_count[6]
+      vertices [V, 18] float32    pos[3], sec[4] (sec.w: flag bits, kept as they are), nrm[3], tex bytes[8]
+      indices [I] float64         block-local
+      transition_vertices / transition_indices   the same for the transition cells, block by block, face by face
+      stats [20] float64          the statistics of the run
+    An array longer than DUMP_ROWS keeps a sample of its rows, in order, drawn with a fixed seed: the same rows for the
+    same length."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    rec = res.records
+    blocks = np.concatenate([np.stack([rec[f] for f in ("level", "coord_id", "id", "vertex_count", "index_count")], axis=1),
+                             rec["trans_vertex_count"], rec["trans_index_count"]], axis=1).astype(np.float64)
+    levels = [res.level(l) for l in range(int(rec["level"].max()) + 1)] if len(rec) else []
+
+    def cat(name, dtype):
+        parts = [getattr(lv, name) for lv in levels]
+        return np.concatenate(parts) if parts else np.zeros(0, dtype)
+
+    def vertex_rows(v):
+        return np.concatenate([v["pos"], v["sec"], v["nrm"], v["tex"].astype(np.float32)], axis=1).astype(np.float32)
+
+    arrays = {"blocks": blocks, "vertices": vertex_rows(cat("verts", res.verts.dtype)), "indices": cat("idx", np.uint32).astype(np.float64),
+              "transition_vertices": vertex_rows(cat("tverts", res.verts.dtype)), "transition_indices": cat("tidx", np.uint32).astype(np.float64)}
+    for name, a in arrays.items():
+        if len(a) > DUMP_ROWS[name]:
+            rows = np.sort(np.random.default_rng(1234).choice(len(a), DUMP_ROWS[name], replace=False))
+            a = a[rows]
+        np.save(os.path.join(directory, name + ".npy"), a)
+    np.save(os.path.join(directory, "stats.npy"), res.stats.astype(np.float64))
 
 
 def measured_peak_hbm():
@@ -343,6 +391,8 @@ def main():
         for _ in range(max(args.warmup, 3)):
             step_resident()
         ms_step = timed(step_resident, args.steps, stream)
+        if args.dump_outputs:
+            dump_outputs(ctx.download(), args.dump_outputs)
         while time.time() - t_load < 1.5:  # keep the load up for at least a few clock samples (50 ms period)
             step_resident()
         clocks = sampler.stop()

@@ -4,15 +4,22 @@ UNMODIFIED reference grid store (src/VoxelGrid.cpp), byte for byte:
   vxb_grid_inject_surface   == Grid::InjectSurface  (+ the returned box)           (:388-488)
   vxb_grid_inject_material  == Grid::InjectMaterial (+ the returned box)           (:490-584)
   vxb_grid_pack             == Grid::PackForSave    (CompressBlock + the blob)     (:610-672, :269-315)
-and the incremental re-polygonization of device-side edits against the reference's incremental Execute."""
+and the incremental re-polygonization of device-side edits against the reference's incremental Execute.
+The reference's grids and blobs are stored as digests (tests/golden/reference_runs.json, made by
+tests/golden/make_golden.py); the incremental test drives the reference itself (oracle/_ref)."""
 import numpy as np
 import pytest
 
 import compare
+import golden_hash
 import harness
 from voxels_b200 import capi
 
 pytestmark = pytest.mark.gpu
+
+
+def stored():
+    return golden_hash.stored("reference_runs.json")["gridstore"]
 
 
 def assert_dense_equal(reference, grid, ctx, what=""):
@@ -25,33 +32,33 @@ def assert_dense_equal(reference, grid, ctx, what=""):
                                  % (what, ch, len(bad), bad[0], a[tuple(bad[0])], b[tuple(bad[0])]))
 
 
-@pytest.mark.parametrize("make,n,start,step", [
+def assert_dense_digest(want, ctx, what=""):
+    assert golden_hash.input_digest(*ctx.download_dense()) == want, "%s: the device grid differs from the reference's" % what
+
+
+FILL_CASES = [
     (lambda n: capi.Surface.sphere((n / 2, n / 2, n / 2), 0.3 * n, 2, 17), 64, (0, 0, 0), 1.0),
     (lambda n: capi.Surface.sphere((10.5, 20.25, 30.0), 19.2), 128, (0, 0, 0), 1.0),
     (lambda n: capi.Surface.plane((0.37, 0.61, 0.7), 40.25, 1, 200), 64, (0, 0, 0), 1.0),
     (lambda n: capi.Surface.sphere((3.0, 4.0, 5.0), 6.5), 32, (-2.0, 1.5, 0.25), 0.375),   # the grid samples world space at start + i * step
     (lambda n: capi.Surface.terrain(n), 128, (0, 0, 0), 1.0),
     (lambda n: capi.Surface.terrain(256, origin=(100, 7), seed=99), 64, (0, 0, 96.0), 1.0),
-])
-def test_fill_equals_reference_constructor(reference, gpu_context, make, n, start, step):
-    s = make(n)
-    g = reference.grid_create_builtin(n, s, start, step)
-    gpu_context.fill(n, s, start, step)
-    assert_dense_equal(reference, g, gpu_context, "fill")
-    reference.grid_destroy(g)
+]
 
 
-def test_fill_terrain_256_equals_host_generator(reference, gpu_context):
-    """the full-size path: device fill vs the multi-threaded host generator (itself pinned to the reference constructor on CPU)"""
-    s = capi.Surface.terrain(256)
-    gpu_context.fill(256, s)
-    got = gpu_context.download_dense()
-    want = reference.builtin_dense(256, s)
-    for a, b in zip(want, got):
-        assert np.array_equal(a, b)
+@pytest.mark.parametrize("make,n,start,step", FILL_CASES)
+def test_fill_equals_reference_constructor(gpu_context, make, n, start, step):
+    gpu_context.fill(n, make(n), start, step)
+    assert_dense_digest(stored()["fill"][FILL_CASES.index((make, n, start, step))], gpu_context, "fill")
 
 
-def _edits(n, count, seed):
+def test_fill_terrain_256_equals_host_generator(gpu_context):
+    """the full-size path: device fill vs the reference constructor of the same surface"""
+    gpu_context.fill(256, capi.Surface.terrain(256))
+    assert_dense_digest(stored()["fill_terrain256"], gpu_context, "fill")
+
+
+def surface_edits(n, count, seed):
     rng = np.random.RandomState(seed)
     out = []
     for i in range(count):
@@ -68,56 +75,61 @@ def _edits(n, count, seed):
     return out
 
 
-def test_inject_surface_equals_reference(reference, gpu_context):
-    n = 64
-    s = capi.Surface.terrain(n)
-    g = reference.grid_create_builtin(n, s)
-    gpu_context.fill(n, s)
-    for i, (pos, ext, surf, kind) in enumerate(_edits(n, 40, 5)):
-        want_box = reference.grid_inject_builtin(g, pos, ext, surf, kind)
-        got_box = gpu_context.inject_surface(pos, ext, surf, kind)
-        assert np.array_equal(want_box, got_box), "edit %d: returned box %s vs %s" % (i, want_box, got_box)
-        assert_dense_equal(reference, g, gpu_context, "edit %d (pos %s ext %s type %d)" % (i, pos, ext, kind))
-    reference.grid_destroy(g)
-
-
-def test_inject_material_equals_reference(reference, gpu_context):
-    n = 64
-    s = capi.Surface.terrain(n)
-    g = reference.grid_create_builtin(n, s)
-    gpu_context.fill(n, s)
-    rng = np.random.RandomState(11)
-    for i in range(30):
+def material_edits(n, count, seed):
+    rng = np.random.RandomState(seed)
+    out = []
+    for i in range(count):
         pos = rng.randint(2, n - 2, size=3).astype(np.float32) if i % 4 else rng.uniform(4, n - 4, size=3).astype(np.float32)
         ext = np.full(3, float(rng.choice([6, 8, 12, 20])), np.float32)
-        material, add = int(rng.randint(0, 5)), bool(i % 2)
-        want_box = reference.grid_inject_material(g, pos, ext, material, add)
+        out.append((pos, ext, int(rng.randint(0, 5)), bool(i % 2)))
+    return out
+
+
+def test_inject_surface_equals_reference(gpu_context):
+    n = 64
+    gpu_context.fill(n, capi.Surface.terrain(n))
+    for i, ((pos, ext, surf, kind), want) in enumerate(zip(surface_edits(n, 40, 5), stored()["inject_surface"])):
+        want_box = np.array(want["box"], np.float32)
+        got_box = gpu_context.inject_surface(pos, ext, surf, kind)
+        assert np.array_equal(want_box, got_box), "edit %d: returned box %s vs %s" % (i, want_box, got_box)
+        assert_dense_digest(want["dense"], gpu_context, "edit %d (pos %s ext %s type %d)" % (i, pos, ext, kind))
+
+
+def test_inject_material_equals_reference(gpu_context):
+    n = 64
+    gpu_context.fill(n, capi.Surface.terrain(n))
+    for i, ((pos, ext, material, add), want) in enumerate(zip(material_edits(n, 30, 11), stored()["inject_material"])):
+        want_box = np.array(want["box"], np.float32)
         got_box = gpu_context.inject_material(pos, ext, material, add)
         assert np.array_equal(want_box, got_box)
-        assert_dense_equal(reference, g, gpu_context, "material edit %d" % i)
-    reference.grid_destroy(g)
+        assert_dense_digest(want["dense"], gpu_context, "material edit %d" % i)
+
+
+def pack_input(name, terrain=None):
+    """(dist, mat, blend) of a packer test; terrain(n) makes the dense terrain of capi.Surface.terrain(n)."""
+    import grids
+    if name == "terrain128":
+        return terrain(128)
+    if name == "zeros32":
+        dist = np.zeros((32, 32, 32), np.int8); mat = np.zeros((32, 32, 32), np.uint8); blend = np.full((32, 32, 32), 255, np.uint8)
+        dist[:, :, 16:] = 3; dist[5, 5, 5] = -1
+        return dist, mat, blend
+    return grids.SMALL[name]()
 
 
 @pytest.mark.parametrize("name", ["terrain128", "hostile64", "noise32", "positive_noise32", "zeros32"])
-def test_pack_equals_reference_pack_for_save(reference, gpu_context, name):
+def test_pack_equals_reference_pack_for_save(gpu_context, name):
     """GPU run-length coding incl. 255-byte run splits, RLE-ineffective (raw) blocks and the BF_Empty flag."""
-    import grids
-    if name == "terrain128":
-        dist, mat, blend = reference.builtin_dense(128, capi.Surface.terrain(128))
-    elif name == "zeros32":
-        dist = np.zeros((32, 32, 32), np.int8); mat = np.zeros((32, 32, 32), np.uint8); blend = np.full((32, 32, 32), 255, np.uint8)
-        dist[:, :, 16:] = 3; dist[5, 5, 5] = -1
-    else:
-        dist, mat, blend = grids.SMALL[name]()
-    g = reference.grid_from_dense(dist, mat, blend)
-    want = reference.grid_pack(g)
-    reference.grid_destroy(g)
+    def terrain(n):
+        gpu_context.fill(n, capi.Surface.terrain(n))
+        return gpu_context.download_dense()
+    dist, mat, blend = pack_input(name, terrain)
+    want = golden_hash.stored("reference_runs.json")["packs"][name]
+    assert golden_hash.input_digest(dist, mat, blend) == want["input_sha256"]
     gpu_context.upload_dense(dist, mat, blend)
     got = gpu_context.pack()
-    assert len(got) == len(want), "blob size %d vs %d" % (len(got), len(want))
-    if not np.array_equal(got, want):
-        bad = np.nonzero(got != want)[0]
-        raise AssertionError("blob differs at %d bytes, first offset %d" % (len(bad), bad[0]))
+    assert len(got) == want["bytes"], "blob size %d vs %d" % (len(got), want["bytes"])
+    assert golden_hash._h(got) == want["sha256"], "blob differs from the reference's Grid::PackForSave"
     # and back: the packed form decodes (on the GPU) to the same voxels
     gpu_context.upload_packed(got)
     back = gpu_context.download_dense()

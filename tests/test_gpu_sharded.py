@@ -96,11 +96,12 @@ def test_virtual_ranks_equal_single_run(gpu_context, name, world, group):
             c.close()
 
 
-def test_sharded_against_reference(reference, gpu_context):
+def test_sharded_against_reference(gpu_context):
+    import golden_hash
     import voxels_b200
     dist, mat, blend = grids.MEDIUM["hostile128"]()
-    g = reference.grid_from_dense(dist, mat, blend)
-    s, _ = reference.polygonize(g)
+    want = golden_hash.reference_run("hostile128")
+    assert golden_hash.input_digest(dist, mat, blend) == want["input_sha256"]
     gpu_context.upload_dense(dist, mat, blend)
     d, m, b = gpu_context.device_pointers()
     contexts = [voxels_b200.Context(0) for _ in range(4)]
@@ -109,17 +110,11 @@ def test_sharded_against_reference(reference, gpu_context):
             c.set_device_grid(128, d, m, b)
         bufs = configure_virtual_ranks(contexts)
         merged, _ = run_virtual_ranks(contexts, bufs)
-        problems = []
-        for l in range(reference.surface_levels(s)):
-            problems += compare.level_diff(reference.surface_level(s, l), merged.level(l), "L%d" % l)
-        if not np.array_equal(reference.surface_stats(s), merged.stats):
-            problems.append("stats differ")
+        problems = golden_hash.run_problems(want, merged, len(want["levels"]))
         assert not problems, "\n".join(problems[:10])
     finally:
         for c in contexts:
             c.close()
-        reference.surface_destroy(s)
-        reference.grid_destroy(g)
 
 
 def _terrain(n):

@@ -1,13 +1,12 @@
-"""CPU tests of the test infrastructure itself (no GPU): the CPU restatement (oracle/restate) is pinned
-  (a) against the unmodified reference compiled under oracle/_ref, when that build is present, and
-  (b) against the committed digests of the reference's output (tests/golden/reference_hashes.json)."""
+"""CPU tests of the test infrastructure itself (no GPU): the CPU restatement (oracle/restate) is pinned against the
+committed digests of the reference's output (tests/golden, made by tests/golden/make_golden.py); the reference's own
+properties are checked against the unmodified reference compiled under oracle/_ref, when that build is present."""
 import json
 import os
 
 import numpy as np
 import pytest
 
-import compare
 import golden_hash
 import grids
 
@@ -19,19 +18,26 @@ def golden():
         return json.load(f)["grids"]
 
 
+class _Restated:
+    """A restatement run seen as a result: .level(l) and .stats."""
+
+    def __init__(self, restatement, h):
+        self.level = lambda l: restatement.level(h, l)
+        self.stats = restatement.stats(h)
+
+
 @pytest.mark.parametrize("name", sorted(grids.SMALL))
-def test_restatement_matches_reference(reference, restatement, name):
+def test_restatement_matches_reference(restatement, name):
     dist, mat, blend = grids.SMALL[name]()
-    g = reference.grid_from_dense(dist, mat, blend)
-    s, _ = reference.polygonize(g, threads=4)
+    want = golden_hash.reference_run(name)
+    assert golden_hash.input_digest(dist, mat, blend) == want["input_sha256"]
     h = restatement.run(dist, mat, blend)
-    assert np.array_equal(reference.grid_empty_flags(g), restatement.empty_flags(h, dist.shape[0])), "BF_Empty rule"
-    assert np.array_equal(reference.surface_stats(s), restatement.stats(h))
-    for l in range(reference.surface_levels(s)):
-        a, b = reference.surface_level(s, l), restatement.level(h, l)
-        assert not compare.level_diff(a, b, "L%d" % l)
-        assert compare.normals_max_ulp(a, b) == 0
-    reference.surface_destroy(s); reference.grid_destroy(g); restatement.destroy(h)
+    flags = golden_hash.stored("reference_runs.json")["empty_flags"][name]
+    assert golden_hash._h(restatement.empty_flags(h, dist.shape[0])) == flags, "BF_Empty rule"
+    assert restatement.levels(h) == len(want["levels"])
+    problems = golden_hash.run_problems(want, _Restated(restatement, h), len(want["levels"]))   # normals: 0 ULP
+    restatement.destroy(h)
+    assert not problems, "\n".join(problems)
 
 
 @pytest.mark.parametrize("name", sorted(grids.SMALL) + ["hostile128"])
@@ -75,15 +81,15 @@ def test_reference_config1_anchors(reference):
     reference.surface_destroy(s); reference.grid_destroy(g)
 
 
-def test_terrain_generator_is_deterministic_and_parity_on_it(reference, restatement):
+def test_terrain_generator_is_deterministic_and_parity_on_it(restatement):
     from voxels_b200 import synth
     d1, m1, b1 = (t.numpy() for t in synth.terrain(64))
     d2, m2, b2 = (t.numpy() for t in synth.terrain(64))
     assert np.array_equal(d1, d2) and np.array_equal(m1, m2) and np.array_equal(b1, b2)
     assert d1.min() == -4 and d1.max() == 4 and set(np.unique(m1)) <= {0, 1, 2, 3}
-    g = reference.grid_from_dense(d1, m1, b1)
-    s, _ = reference.polygonize(g, threads=4)
+    want = golden_hash.reference_run("terrain64")
+    assert golden_hash.input_digest(d1, m1, b1) == want["input_sha256"]
     h = restatement.run(d1, m1, b1)
-    for l in range(reference.surface_levels(s)):
-        assert not compare.level_diff(reference.surface_level(s, l), restatement.level(h, l), "L%d" % l)
-    reference.surface_destroy(s); reference.grid_destroy(g); restatement.destroy(h)
+    problems = golden_hash.run_problems(want, _Restated(restatement, h), len(want["levels"]), stats=False)
+    restatement.destroy(h)
+    assert not problems, "\n".join(problems)

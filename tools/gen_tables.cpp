@@ -1,60 +1,47 @@
-// Build-time generator: reads the Transvoxel look-up tables from the reference checkout
-// (-DVXB_TABLES_INL="<path>/src/Transvoxel.inl", included, never copied into this repo) and
-// prints them re-packed for the device (byte/ushort arrays, fixed strides) as a C header.
-// Run by voxels_b200/build.py; output goes to build/gen/vxb_tables_data.h (git-ignored).
+// Regenerates tests/golden/transvoxel_tables.bin from a checkout of the reference
+// (-DVXB_TABLES_INL="<path>/src/Transvoxel.inl", included, never copied into this repo):
+//
+//   g++ -O1 -w -DVXB_TABLES_INL='"<reference>/src/Transvoxel.inl"' tools/gen_tables.cpp -o gen_tables
+//   ./gen_tables > tests/golden/transvoxel_tables.bin
+//
+// The file holds the Transvoxel look-up tables re-packed for the device (byte/ushort arrays, fixed strides,
+// little endian), in the order and sizes of voxels_b200/build.py TABLES_LAYOUT; build.py turns it into the
+// C header the kernels and the CPU restatement include (build/gen/vxb_tables_data.h).
 #include <cstdio>
 #include <cstdint>
 #include VXB_TABLES_INL
 
-static uint64_t g_Hash = 1469598103934665603ull; // FNV-1a over every emitted value (little endian)
-static void hashByte(unsigned v) { g_Hash ^= (v & 0xFF); g_Hash *= 1099511628211ull; }
-
-static void emit8(const char* name, const unsigned char* data, size_t count)
+static void emit8(const unsigned char* data, size_t count)
 {
-	printf("VXB_TABLE_QUAL const unsigned char VXB_TABLE_NAME(%s)[%zu] = {", name, count);
-	for (size_t i = 0; i < count; ++i) { printf("%s%u,", (i % 32) ? "" : "\n\t", data[i]); hashByte(data[i]); }
-	printf("\n};\n\n");
+	fwrite(data, 1, count, stdout);
 }
 
-static void emit16(const char* name, const unsigned short* data, size_t count)
+static void emit16(const unsigned short* data, size_t count)
 {
-	printf("VXB_TABLE_QUAL const unsigned short VXB_TABLE_NAME(%s)[%zu] = {", name, count);
-	for (size_t i = 0; i < count; ++i) { printf("%s0x%04X,", (i % 12) ? "" : "\n\t", data[i]); hashByte(data[i]); hashByte(data[i] >> 8); }
-	printf("\n};\n\n");
+	for (size_t i = 0; i < count; ++i) { putchar(data[i] & 0xFF); putchar(data[i] >> 8); }
 }
 
 int main()
 {
-	printf("// GENERATED by tools/gen_tables.cpp from the reference's src/Transvoxel.inl - do not edit, do not commit.\n");
-	printf("//\n");
-	printf("// The following data originates from Eric Lengyel's Transvoxel Algorithm.\n");
-	printf("// http://www.terathon.com/voxels/\n");
-	printf("//\n");
-	printf("// Packing: cell data rows are {geometryCounts, vertexIndex[...]} with strides 16 (regular) and 40 (transition).\n");
-	printf("// May be included more than once with different VXB_TABLE_QUAL / VXB_TABLE_NAME (e.g. __constant__ and __device__ copies).\n");
-	printf("#ifndef VXB_TABLE_QUAL\n#define VXB_TABLE_QUAL static\n#endif\n#ifndef VXB_TABLE_NAME\n#define VXB_TABLE_NAME(x) vxb##x\n#endif\n\n");
-
-	emit8("RegularCellClass", regularCellClass, 256);
+	emit8(regularCellClass, 256);
 
 	unsigned char reg[16 * 16];
 	for (int c = 0; c < 16; ++c) {
 		reg[c * 16] = regularCellData[c].geometryCounts;
 		for (int i = 0; i < 15; ++i) reg[c * 16 + 1 + i] = regularCellData[c].vertexIndex[i];
 	}
-	emit8("RegularCellData", reg, sizeof(reg));
-	emit16("RegularVertexData", &regularVertexData[0][0], 256 * 12);
+	emit8(reg, sizeof(reg));
+	emit16(&regularVertexData[0][0], 256 * 12);
 
-	emit8("TransitionCellClass", transitionCellClass, 512);
+	emit8(transitionCellClass, 512);
 	unsigned char trans[56 * 40];
 	for (int c = 0; c < 56; ++c) {
 		for (int i = 0; i < 40; ++i) trans[c * 40 + i] = 0;
 		trans[c * 40] = (unsigned char)transitionCellData[c].geometryCounts;
 		for (int i = 0; i < 36; ++i) trans[c * 40 + 1 + i] = transitionCellData[c].vertexIndex[i];
 	}
-	emit8("TransitionCellData", trans, sizeof(trans));
-	emit8("TransitionCornerData", transitionCornerData, 13);
-	emit16("TransitionVertexData", &transitionVertexData[0][0], 512 * 12);
-
-	printf("#ifndef VXB_TABLES_FNV1A\n#define VXB_TABLES_FNV1A 0x%016llXull\n#endif\n", (unsigned long long)g_Hash);
+	emit8(trans, sizeof(trans));
+	emit8(transitionCornerData, 13);
+	emit16(&transitionVertexData[0][0], 512 * 12);
 	return 0;
 }
